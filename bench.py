@@ -2,7 +2,7 @@
 """bench.py -- X25519 scalar-mults/s on N B200s (BASELINE.json metric), with the INT32-IMAD
 roofline, the end-to-end (host buffers, C ABI) figure and the reference's CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--keys 1048576] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--keys 1048576] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (rfc7748: clamp, import, 255 ladder steps, inversion,
 export) over one batch of 2^20 random raw key/point pairs per GPU (BASELINE configs[1]).
@@ -51,7 +51,17 @@ def parse():
     ap.add_argument("--parity-keys", type=int, default=-1,
                     help="keys of EVERY rank's first step checked against the reference build before timing "
                          "(-1 = all local keys, capped at 2^20 per rank)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the X25519 results of the last one to DIR/x25519_out.npy "
+                         "([rows, 32] byte values as float32; every key up to 2^18, beyond that a fixed seeded sample "
+                         "of 2^18 keys, see dump_rows); with several GPUs, an equal seeded sample of every GPU's "
+                         "keys, in key order")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; --impl reference has none")
+    return args
 
 
 # ------------------------------------------------------------------------------------------
@@ -72,6 +82,31 @@ def make_inputs(n, seed):
     import numpy as np
     rng = np.random.Generator(np.random.PCG64(seed))
     return rng.integers(0, 256, (n, NB), dtype=np.uint8), rng.integers(0, 256, (n, NB), dtype=np.uint8)
+
+
+DUMP_ROWS = 1 << 18          # 2^18 keys x 32 bytes as float32 = 32 MiB
+
+
+def dump_rows(n, m=DUMP_ROWS):
+    """Rows of an n-key shard that --dump-outputs writes: all of them up to m, else a fixed seeded sample of m in
+    ascending order, so that two builds run with the same arguments write the same rows."""
+    import numpy as np
+    if n <= m:
+        return np.arange(n)
+    return np.sort(np.random.Generator(np.random.PCG64(2020)).choice(n, m, replace=False))
+
+
+def dump_part(out, shards):
+    """The rows of one GPU's [n, 32] uint8 result that --dump-outputs writes when `shards` GPUs share the batch."""
+    import torch
+    return out[torch.from_numpy(dump_rows(out.shape[0], DUMP_ROWS // shards)).to(out.device)]
+
+
+def dump_outputs(path, parts):
+    """parts: dump_part of every GPU's result of the last timed step, in key order."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "x25519_out.npy"), np.concatenate([p.cpu().numpy() for p in parts]).astype(np.float32))
 
 
 def load_reference():
@@ -502,6 +537,8 @@ def run_single_process(args):
     sync()
     wall = time.perf_counter() - t0
     ms = max(e0.elapsed_time(e1) for e0, e1 in ev)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [dump_part(dv[g], N) for g in range(N)])
     # parity of every device's shard against the reference build (set of the last step)
     ref = load_reference()
     parity, pn = None, 0
@@ -635,6 +672,13 @@ def main():
     t_end = time.time()
     ms = e0.elapsed_time(e1)
     launches = args.steps
+    if args.dump_outputs:
+        parts = [dump_part(dv[(args.steps - 1) % NSETS], world)]
+        if world > 1:
+            parts = [torch.empty_like(parts[0]) for _ in range(world)]
+            dist.all_gather(parts, dump_part(dv[(args.steps - 1) % NSETS], world))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, parts)
 
     # ---- end to end: host buffers through the C ABI (H2D + ladder + D2H inside the timed region) --
     # The buffers are pinned, so the library takes its zero-copy route: one launch whose threads read the

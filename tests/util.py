@@ -58,6 +58,13 @@ def random_bytes(seed, n, nb):
     return rng.integers(0, 256, (n, nb), dtype=np.uint8)
 
 
+def sample_rows(n, m, head=0):
+    """Rows checked against the restatements where the reference build (oracle/_ref) is absent: the first `head`
+    rows (planted corner cases) and a fixed seeded sample of m of the others, ascending."""
+    rest = np.random.Generator(np.random.PCG64(n)).choice(np.arange(head, n), min(m, n - head), replace=False)
+    return np.concatenate([np.arange(head), np.sort(rest)])
+
+
 def ref_rfc7748_batch(lib, k, u):
     out = np.zeros_like(k)
     lib.ref_rfc7748_batch(k.ctypes.data_as(ctypes.c_char_p), u.ctypes.data_as(ctypes.c_char_p),
