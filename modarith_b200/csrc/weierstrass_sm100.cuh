@@ -179,6 +179,24 @@ template <class F> struct Weierstrass {
     inf(O);
     cmv(bad, O, P);
   }
+  // set() that reports what it checked: 1 iff xw < p, yw < p and (x, y) is on the curve (public-key validation,
+  // SEC1 v2 section 3.2.2.1); P is O otherwise.  set() keeps modimp semantics (a coordinate >= p reduces).
+  static MAB_DEV uint32_t set_checked(Pt& P, const uint32_t (&xw)[L], const uint32_t (&yw)[L]) {
+    uint32_t v[L], t[L], b[L];
+    const uint32_t lt = Fd::from_words(P.x, xw) & Fd::from_words(P.y, yw);
+    F::sqr(v, P.x);
+    F::mul(v, v, P.x);
+    F::sub(v, v, P.x); F::sub(v, v, P.x); F::sub(v, v, P.x);
+    F::set_b(b);
+    F::add(v, v, b);
+    F::sqr(t, P.y);
+    const uint32_t on = Fd::cmp(t, v);
+    Fd::one(P.z);
+    Pt O;
+    inf(O);
+    cmv(1u - on, O, P);
+    return lt & on;
+  }
 
   // ecnXXXget (weierstrass.c:297-349): affine coordinates as canonical plain words; O -> (0, 1)
   static MAB_DEV void get(uint32_t (&xw)[L], uint32_t (&yw)[L], const Pt& P) {

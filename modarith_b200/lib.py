@@ -168,6 +168,8 @@ def load() -> ctypes.CDLL:
         fn.restype = c_int
     for P in CURVES:
         _bind_curve(lib, P)
+    lib.mab_NIST256_ecdsa_verify.argtypes = [_P] * 6 + [c_size_t, c_void_p]
+    lib.mab_NIST256_ecdsa_verify.restype = c_int
     _lib = lib
     return lib
 
@@ -183,6 +185,11 @@ def exported_symbols():
         syms += ["mab_%s_rfc7748" % P, "mab_%s_rfc7748_host" % P, "mab_%s_rfc7748_validate" % P,
                  "mab_%s_rfc7748_perkey" % P, "mab_%s_rfc7748_host_multi" % P]
     return syms
+
+
+def signature_symbols():
+    """Every symbol include/modarith_b200_sig.h declares."""
+    return ["mab_NIST256_ecdsa_verify"]
 
 
 def check(code: int, what: str = "", lib=None):

@@ -14,6 +14,9 @@ converter (`parse.py`), restated for batches:
   `x448_test.json`: `testGroups[].tests[]` with `public`, `private`, `shared`, `result`) into the
   byte arrays `rfc7748()` takes and push the whole suite through the batch ladder in one call --
   the "external vector suites through the batch API" use the survey names.
+* `load_ecdsa_vectors` / `run_ecdsa_vectors` do the same for Wycheproof ECDSA verification files
+  (`EcdsaVerify` groups with DER signatures, `EcdsaP1363Verify` groups with r || s; secp256r1 only) through
+  `modarith_b200.ecdsa`.
 
 Host-side format code only: nothing here computes field arithmetic.
 """
@@ -26,7 +29,8 @@ from typing import Iterable, List, Sequence
 import numpy as np
 
 __all__ = ["from_hex", "to_hex", "reverse", "parse_signature_vectors", "signature_lines",
-           "SignatureVector", "XdhVector", "load_xdh_vectors", "run_xdh_vectors"]
+           "SignatureVector", "XdhVector", "load_xdh_vectors", "run_xdh_vectors", "EcdsaVector", "load_ecdsa_vectors",
+           "run_ecdsa_vectors"]
 
 _HEXVAL = np.zeros(256, dtype=np.uint8)
 for _c in range(256):
@@ -191,6 +195,75 @@ def run_xdh_vectors(curve: str, vectors: Sequence[XdhVector], device=None):
             passed[i] = bool(same[gi])
         gi += 1
     return bv, passed
+
+
+# ---------------------------------------------------------------------------------------------
+# ECDSA P-256 suites through the batch verifier
+# ---------------------------------------------------------------------------------------------
+@dataclass
+class EcdsaVector:
+    tc_id: int
+    comment: str
+    msg: str
+    sig: str
+    result: str
+    flags: tuple
+    public_key: str          # SEC1 uncompressed, hex
+    hash: str                # hashlib name; None when `msg` is the digest itself (groups marked "prehashed")
+    encoding: str            # "der" or "p1363"
+
+
+_ECDSA_GROUPS = {"EcdsaVerify": "der", "EcdsaP1363Verify": "p1363"}
+
+
+def _hashlib_name(sha: str) -> str:
+    """Wycheproof's "SHA-256", "SHA3-256", "SHA-512/256" -> hashlib's "sha256", "sha3_256", "sha512_256"."""
+    return sha.lower().replace("sha3-", "sha3_").replace("/", "_").replace("-", "")
+
+
+def load_ecdsa_vectors(source) -> List[EcdsaVector]:
+    """The secp256r1 tests of a Wycheproof ECDSA verification file (ecdsa_verify_schema / ecdsa_p1363_verify_schema):
+    accepts a path, JSON text or a parsed dict.  Groups on other curves or of other types are left out.  A group
+    with `"prehashed": true` carries the digest itself in `msg` (rows no message can produce, such as digest 0)."""
+    if isinstance(source, dict):
+        doc = source
+    else:
+        s = str(source)
+        doc = json.loads(s) if s.lstrip().startswith("{") else json.load(open(s))
+    out = []
+    for g in doc.get("testGroups", []):
+        enc = _ECDSA_GROUPS.get(g.get("type"))
+        key = g.get("publicKey") or g.get("key") or {}
+        if enc is None or key.get("curve") != "secp256r1":
+            continue
+        h = None if g.get("prehashed") else _hashlib_name(g["sha"])
+        for t in g.get("tests", []):
+            out.append(EcdsaVector(int(t.get("tcId", len(out) + 1)), t.get("comment", ""), t["msg"], t["sig"],
+                                   t.get("result", "valid"), tuple(t.get("flags", ())), key["uncompressed"], h, enc))
+    return out
+
+
+def run_ecdsa_vectors(vectors: Sequence[EcdsaVector]):
+    """All vectors of a suite in ONE call of the batch verifier.  A "valid" test passes when the signature verifies,
+    an "invalid" one when it does not; "acceptable" tests (legacy encodings a verifier may accept or reject) always
+    pass and are reported by the caller.  Returns (verified bool[n], passed bool[n])."""
+    from .ecdsa import prepare, verify_digest
+
+    n = len(vectors)
+    rows = np.zeros((5, n, 32), dtype=np.uint8)
+    parsed = np.zeros(n, dtype=bool)
+    kinds = sorted({(v.hash or "", v.encoding) for v in vectors})
+    for h, enc in kinds:
+        idx = [i for i, v in enumerate(vectors) if (v.hash or "", v.encoding) == (h, enc)]
+        part, ok = prepare([bytes.fromhex(vectors[i].msg) for i in idx], [bytes.fromhex(vectors[i].sig) for i in idx],
+                           [bytes.fromhex(vectors[i].public_key) for i in idx], h or None, enc)
+        for k in range(5):
+            rows[k, idx] = part[k]
+        parsed[idx] = ok
+    verified = (verify_digest(*rows) & parsed) if n else parsed
+    want = np.array([v.result == "valid" for v in vectors], dtype=bool)
+    passed = (verified == want) | np.array([v.result == "acceptable" for v in vectors], dtype=bool)
+    return verified, passed
 
 
 def main(argv=None):
