@@ -22,6 +22,18 @@ extern "C" {
 MAB_API int mab_NIST256_ecdsa_verify(const char *h, const char *r, const char *s, const char *qx, const char *qy,
                                      unsigned char *ok, size_t n, void *stream);
 
+/* Ed25519 (RFC 8032 section 5.1.7, pure Ed25519, the cofactorless equation), one signature per row; byte strings
+ * as RFC 8032 encodes them (little-endian), row i at offset 64*i (h, sig) or 32*i (pk):
+ *   h        SHA-512(R || A || M), 64 bytes, reduced mod L here
+ *   sig      R || S, 64 bytes; rows with S >= L are invalid; R is compared as bytes with the encoding of
+ *            [S]B - [k]A (all 256 bits), never decoded
+ *   pk       the public key A, 32 bytes; rows whose A does not decode strictly (y >= p, no square root,
+ *            x = 0 with the sign bit set) are invalid
+ * Small-order A and R are accepted where the equation holds.  ok[i] = 1 if row i is a valid signature, 0 if not.
+ * Every row does the same work whatever its inputs.  n = 0 is a no-op. */
+MAB_API int mab_ED25519_eddsa_verify(const char *h, const char *sig, const char *pk, unsigned char *ok,
+                                     size_t n, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

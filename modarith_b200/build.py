@@ -72,8 +72,8 @@ def _nvcc():
 def _digest():
     h = hashlib.sha256()
     h.update(" ".join(NVCC_FLAGS).encode())
-    roots = [CSRC, os.path.join(CSRC, "gen"), os.path.join(PKG, "..", "include")]
-    for root in roots:
+    roots = [CSRC, os.path.join(CSRC, "gen"), os.path.join(OBJDIR, "gen"), os.path.join(PKG, "..", "include")]
+    for root in filter(os.path.isdir, roots):
         for fn in sorted(os.listdir(root)):
             p = os.path.join(root, fn)
             if os.path.isfile(p) and fn.endswith((".cu", ".cuh", ".inc", ".h")):

@@ -114,4 +114,68 @@ template <class F> struct Edwards {
     Fd::to_words(xw, x);
     Fd::to_words(yw, y);
   }
+
+  // Point decoding of RFC 8032 section 5.1.3, strict: enc = y (low 255 bits) | sign of x << 255, little-endian
+  // words.  1 iff y < p, x^2 = (y^2 - 1) / (d y^2 + 1) has a root and not (x = 0 with the sign bit set); P is the
+  // point (coordinates tight, as set() leaves them) where ok = 1 and O elsewhere.  One progenitor chain:
+  // x = u v^3 (u v^7)^((p-5)/8), then x *= sqrt(-1) where v x^2 = -u (p = 5 mod 8).  Every check is a mask.
+  static MAB_DEV uint32_t decode(Pt& P, const uint32_t (&enc)[L]) {
+    static_assert(F::PM1D2 == 2, "the (p-5)/8 square-root chain needs p = 5 mod 8");
+    uint32_t yw[L], y[L], u[L], v[L], t[L], x[L], w[L], one[L];
+#pragma unroll
+    for (int j = 0; j < L; j++) yw[j] = enc[j];
+    const uint32_t sgn = yw[L - 1] >> 31;
+    yw[L - 1] &= 0x7fffffffu;
+    uint32_t ok = Fd::from_words(y, yw);
+    Fd::one(one);
+    F::sqr(u, y);
+    F::set_ed_d(t);
+    F::mul(v, u, t);
+    F::add(v, v, one);                             // v = d y^2 + 1 (never 0: d is a non-square)
+    F::sub(u, u, one);                             // u = y^2 - 1
+    F::sqr(t, v);
+    F::mul(t, t, v);                               // v^3
+    F::mul(x, u, t);                               // u v^3
+    F::sqr(t, t);
+    F::mul(t, t, v);                               // v^7
+    F::mul(t, t, u);                               // u v^7
+    F::pro(w, t);                                  // (u v^7)^((p-5)/8)
+    F::mul(x, x, w);
+    F::sqr(t, x);
+    F::mul(t, t, v);                               // v x^2
+    const uint32_t is_u = Fd::cmp(t, u);
+    F::neg(w, u);
+    const uint32_t is_neg_u = Fd::cmp(t, w);
+    F::set_roi(w);
+    F::mul(t, x, w);
+    Fd::cmv(is_neg_u, t, x);
+    ok &= is_u | is_neg_u;
+    uint32_t xc[L];
+    Fd::to_words(xc, x);
+    uint32_t nz = 0;
+#pragma unroll
+    for (int j = 0; j < L; j++) nz |= xc[j];
+    ok &= 1u - (sgn & (nz == 0 ? 1u : 0u));
+    F::neg(t, x);
+    Fd::cmv((xc[0] & 1u) ^ sgn, t, x);
+    F::mul(P.x, x, one);                           // products: tight whatever neg / import left
+    F::mul(P.y, y, one);
+    Fd::one(P.z);
+    Pt O;
+    inf(O);
+    cmv(1u - ok, O, P);
+    return ok;
+  }
+
+  // Point encoding (RFC 8032 section 5.1.2): canonical y with the low bit of x in bit 255, little-endian words.
+  // One inversion of Z (Z != 0 for every point the complete formulas produce).
+  static MAB_DEV void encode(uint32_t (&enc)[L], const Pt& P) {
+    uint32_t i[L], x[L], y[L], xw[L];
+    Fd::template inv<false>(i, P.z, P.z);
+    F::mul(x, P.x, i);
+    F::mul(y, P.y, i);
+    Fd::to_words(xw, x);
+    Fd::to_words(enc, y);
+    enc[L - 1] |= xw[0] << 31;
+  }
 };

@@ -4,7 +4,7 @@ from __future__ import annotations
 import argparse
 import os
 
-from ..primes import PRIMES, ALL_PRIMES, Prime
+from ..primes import PRIMES, ALL_PRIMES, ORDER_PRIMES, Prime
 from .plan import make_plan
 from .emit import emit_field_header
 
@@ -14,6 +14,8 @@ CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "csrc")
 def resolve(prime: str, family: str) -> Prime:
     if prime in ALL_PRIMES:
         return ALL_PRIMES[prime]
+    if prime in ORDER_PRIMES:
+        return ORDER_PRIMES[prime]
     if prime[0].isdigit():                      # expression, as pseudo.py:1553-1556
         p = eval(prime, {"__builtins__": {}})
         return Prime("P%d" % p.bit_length(), p, family)
@@ -53,7 +55,14 @@ def main(family: str, argv) -> int:
     return 0
 
 
+BUILD_GEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "build", "gen")
+
+
 def generate_all(verbose=False, outdir=None):
-    """Headers of every built-in modulus; into csrc/gen (the committed copies) or, for tests, into `outdir`/gen."""
-    return [generate(P, None if outdir is None else os.path.join(outdir, "gen", "field_%s.cuh" % P.name), verbose=verbose)
-            for P in ALL_PRIMES.values()]
+    """Headers of every built-in modulus into csrc/gen (the committed copies) and of the group orders in ORDER_PRIMES
+    into the build directory's gen/ (made at build time, not committed; the build's include path has the build
+    directory); or, for tests, all of them into `outdir`/gen."""
+    out = [generate(P, None if outdir is None else os.path.join(outdir, "gen", "field_%s.cuh" % P.name), verbose=verbose)
+           for P in ALL_PRIMES.values()]
+    gen = BUILD_GEN if outdir is None else os.path.join(outdir, "gen")
+    return out + [generate(P, os.path.join(gen, "field_%s.cuh" % P.name), verbose=verbose) for P in ORDER_PRIMES.values()]

@@ -170,6 +170,8 @@ def load() -> ctypes.CDLL:
         _bind_curve(lib, P)
     lib.mab_NIST256_ecdsa_verify.argtypes = [_P] * 6 + [c_size_t, c_void_p]
     lib.mab_NIST256_ecdsa_verify.restype = c_int
+    lib.mab_ED25519_eddsa_verify.argtypes = [_P] * 4 + [c_size_t, c_void_p]
+    lib.mab_ED25519_eddsa_verify.restype = c_int
     _lib = lib
     return lib
 
@@ -189,7 +191,7 @@ def exported_symbols():
 
 def signature_symbols():
     """Every symbol include/modarith_b200_sig.h declares."""
-    return ["mab_NIST256_ecdsa_verify"]
+    return ["mab_NIST256_ecdsa_verify", "mab_ED25519_eddsa_verify"]
 
 
 def check(code: int, what: str = "", lib=None):

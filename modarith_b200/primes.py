@@ -86,6 +86,12 @@ NIST256ORDER = Prime("NIST256ORDER", 0xFFFFFFFF00000000FFFFFFFFFFFFFFFFBCE6FAADA
 EXTRA_PRIMES = {q.name: q for q in (SECP256K1, NIST256ORDER)}
 ALL_PRIMES = dict(PRIMES, **EXTRA_PRIMES)
 
+# group orders whose field code is compiled only INTO another modulus' unit (no entry points of their own, no
+# mab_<NAME>_* symbols): the Ed25519 group order L, for k = SHA-512(R || A || M) mod L and the S < L check of
+# Ed25519 verification (csrc/eddsa_sm100.cuh, included by mab_capi_X25519.cu)
+ED25519ORDER = Prime("ED25519ORDER", 2**252 + 27742317777372353535851937790883648493, "monty")
+ORDER_PRIMES = {q.name: q for q in (ED25519ORDER,)}
+
 # Every other named modulus of the reference's tables (pseudo.py:1487-1550 "pseudo", monty.py:1961-2108 "monty"),
 # as data: none of them is compiled into the shipped library, `python -m modarith_b200.build --prime NAME` builds an
 # add-on library for one (libmodarith_b200_<NAME>.so, same C ABI; Field(NAME) finds it).  A name both generators

@@ -17,6 +17,8 @@ converter (`parse.py`), restated for batches:
 * `load_ecdsa_vectors` / `run_ecdsa_vectors` do the same for Wycheproof ECDSA verification files
   (`EcdsaVerify` groups with DER signatures, `EcdsaP1363Verify` groups with r || s; secp256r1 only) through
   `modarith_b200.ecdsa`.
+* `load_eddsa_vectors` / `run_eddsa_vectors` do the same for Wycheproof EdDSA verification files (`EddsaVerify`
+  groups on edwards25519) through `modarith_b200.eddsa`.
 
 Host-side format code only: nothing here computes field arithmetic.
 """
@@ -30,7 +32,7 @@ import numpy as np
 
 __all__ = ["from_hex", "to_hex", "reverse", "parse_signature_vectors", "signature_lines",
            "SignatureVector", "XdhVector", "load_xdh_vectors", "run_xdh_vectors", "EcdsaVector", "load_ecdsa_vectors",
-           "run_ecdsa_vectors"]
+           "run_ecdsa_vectors", "EddsaVector", "load_eddsa_vectors", "run_eddsa_vectors"]
 
 _HEXVAL = np.zeros(256, dtype=np.uint8)
 for _c in range(256):
@@ -261,6 +263,53 @@ def run_ecdsa_vectors(vectors: Sequence[EcdsaVector]):
             rows[k, idx] = part[k]
         parsed[idx] = ok
     verified = (verify_digest(*rows) & parsed) if n else parsed
+    want = np.array([v.result == "valid" for v in vectors], dtype=bool)
+    passed = (verified == want) | np.array([v.result == "acceptable" for v in vectors], dtype=bool)
+    return verified, passed
+
+
+# ---------------------------------------------------------------------------------------------
+# Ed25519 suites through the batch verifier
+# ---------------------------------------------------------------------------------------------
+@dataclass
+class EddsaVector:
+    tc_id: int
+    comment: str
+    msg: str
+    sig: str
+    result: str
+    flags: tuple
+    public_key: str          # the 32-byte encoding A, hex
+
+
+def load_eddsa_vectors(source) -> List[EddsaVector]:
+    """The edwards25519 tests of a Wycheproof EdDSA verification file (eddsa_verify_schema): accepts a path, JSON
+    text or a parsed dict.  The key is `publicKey.pk` (or `key.pk` in older files); groups on other curves (Ed448)
+    or of other types are left out."""
+    if isinstance(source, dict):
+        doc = source
+    else:
+        s = str(source)
+        doc = json.loads(s) if s.lstrip().startswith("{") else json.load(open(s))
+    out = []
+    for g in doc.get("testGroups", []):
+        key = g.get("publicKey") or g.get("key") or {}
+        if g.get("type") != "EddsaVerify" or key.get("curve") != "edwards25519":
+            continue
+        for t in g.get("tests", []):
+            out.append(EddsaVector(int(t.get("tcId", len(out) + 1)), t.get("comment", ""), t["msg"], t["sig"],
+                                   t.get("result", "valid"), tuple(t.get("flags", ())), key["pk"]))
+    return out
+
+
+def run_eddsa_vectors(vectors: Sequence[EddsaVector]):
+    """All vectors of a suite in ONE call of the batch verifier.  A "valid" test passes when the signature verifies,
+    an "invalid" one when it does not; "acceptable" tests always pass and are reported by the caller.  Returns
+    (verified bool[n], passed bool[n])."""
+    from .eddsa import verify
+
+    verified = verify([bytes.fromhex(v.msg) for v in vectors], [bytes.fromhex(v.sig) for v in vectors],
+                      [bytes.fromhex(v.public_key) for v in vectors])
     want = np.array([v.result == "valid" for v in vectors], dtype=bool)
     passed = (verified == want) | np.array([v.result == "acceptable" for v in vectors], dtype=bool)
     return verified, passed

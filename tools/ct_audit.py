@@ -34,6 +34,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "modarith_b200", "build")
 DEFAULT = [("mab_capi_X25519.o", "k_rfc7748"), ("mab_capi_X448.o", "k_rfc7748"),
            ("mab_capi_NIST256.o", "k_ecnmul"), ("mab_capi_X25519.o", "k_ecnmul"), ("mab_capi_NIST256.o", "k_ecdsa"),
+           ("mab_capi_X25519.o", "k_eddsa"),
            ("mab_capi_NIST256.o", "k_field"), ("mab_capi_X25519.o", "k_field"), ("mab_capi_X448.o", "k_field"),
            ("mab_capi_SECP256K1.o", "k_field"), ("mab_capi_NIST256ORDER.o", "k_field"),
            ("mab_capi_NIST256.o", "k_inv_shared"), ("mab_capi_X25519.o", "k_inv_shared"),
