@@ -19,7 +19,9 @@
 enum SimOp {
   S_ADD, S_SUB, S_NEG, S_MUL, S_SQR, S_MLI, S_NSQR, S_PRO, S_INV, S_INVH, S_QR, S_QRH, S_SQRT, S_SQRTH,
   S_IS1, S_IS0, S_ONE, S_INT, S_NRES, S_REDC, S_CSW, S_CMV, S_SHL, S_SHR, S_HAF, S_2R, S_SIGN, S_CMP, S_FSB,
-  S_IMPW, S_EXPW
+  S_IMPW, S_EXPW,
+  // the generated blocks on their own, on any stored words (tests/test_gpu_blocks.py)
+  S_MLA, S_ADDTT, S_SUBTT, S_MULW, S_SQRW, S_CANON, S_REDCW
 };
 
 template <class F> static int sim_op(int op, const uint32_t* pa, const uint32_t* pb, uint32_t scalar, uint32_t* pr, uint32_t* pr2) {
@@ -60,6 +62,13 @@ template <class F> static int sim_op(int op, const uint32_t* pa, const uint32_t*
     case S_FSB: Fd::cpy(r, a); ret = (int)Fd::fsb(r); break;
     case S_IMPW: ret = (int)Fd::from_words(r, a); break;
     case S_EXPW: Fd::to_words(r, a); break;
+    case S_MLA: F::mla(r, a, scalar, b); break;
+    case S_ADDTT: F::add_tt(r, a, b); break;
+    case S_SUBTT: F::sub_tt(r, a, b); break;
+    case S_MULW: F::mul_w(r, a, b); break;
+    case S_SQRW: F::sqr_w(r, a); break;
+    case S_CANON: ret = (int)F::canon(r, a); break;
+    case S_REDCW: F::redc(r, a); break;
     default: return -1;
   }
   for (int i = 0; i < L; i++) pr[i] = r[i];

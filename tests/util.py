@@ -8,7 +8,7 @@ from modarith_b200.primes import ALL_PRIMES as PRIMES
 
 SIM_OPS = ["ADD", "SUB", "NEG", "MUL", "SQR", "MLI", "NSQR", "PRO", "INV", "INVH", "QR", "QRH", "SQRT", "SQRTH",
            "IS1", "IS0", "ONE", "INT", "NRES", "REDC", "CSW", "CMV", "SHL", "SHR", "HAF", "2R", "SIGN", "CMP", "FSB",
-           "IMPW", "EXPW"]
+           "IMPW", "EXPW", "MLA", "ADDTT", "SUBTT", "MULW", "SQRW", "CANON", "REDCW"]
 SIM = {n: i for i, n in enumerate(SIM_OPS)}
 
 
